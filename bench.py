@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — frames/s through detect -> match -> local BA at 1920x1080 mono (BASELINE.json metric), one JSON line.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step is one frame through the whole hot path: ORB extract (2000 kp) of a NEW 1080p frame, 256-bit Hamming match against the
 previous frame's descriptors, and one local bundle adjustment (50 keyframes / 2000 landmarks / 10 000 observations, 10 LM
@@ -18,14 +18,18 @@ iterations, 50-iteration block-Jacobi PCG cap).
                all-reduce of the compact reduced camera system per LM iteration -- STRONG scaling (total work fixed).
 N>1 for the per-frame path: independent replicas, one rank per GPU, no data-path collective -> weak scaling.
 
-The timed block of K steps is repeated (each repetition bracketed by barrier + synchronize, max over ranks) and the MEDIAN block is
-reported, so that a 20-step run is not a 24 ms coin flip; the clock sampler starts before the warm-up.
+The timed block is exactly K steps (bracketed by barrier + synchronize, max over ranks); the clock sampler starts before the warm-up.
+The default 1000 steps time about a second (1.08 ms per step on a B200 at a 1000 W power limit): a much shorter window would show
+clock ramp and scheduler noise in the one number reported.
+
+--dump-outputs DIR writes what the pipelined timed path computed in its last step, as a caller of that path receives it, to DIR/<name>.npy
+(float32 / float64): the keypoints and descriptors of the last frame, its matches against the previous frame and the local BA window's
+poses, points and costs.  The inputs depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
 import json
-import math
 import os
 import queue
 import subprocess
@@ -175,6 +179,21 @@ def cpu_path(frames, ba_problem, steps, threads):
     return steps / dt, what
 
 
+def dump_outputs(out_dir, feats, graph, res):
+    """The last timed step's results, as Features.download / Features.matches / BAGraph.download and the BaResult give them."""
+    from gslam_b200.capi import KP_DTYPE
+    kps, desc = feats.download()
+    idx, d1, d2 = feats.matches()
+    poses, points = graph.download()
+    out = {"keypoints": np.stack([kps[f].astype(np.float32) for f in KP_DTYPE.names], axis=1),   # x y size angle response octave class_id
+           "descriptors": desc.astype(np.float32), "match_train_index": idx.astype(np.float32), "match_distance": d1.astype(np.float32),
+           "match_second_distance": d2.astype(np.float32), "ba_poses_wc": poses, "ba_points": points,
+           "ba_cost": np.array([res.initial_cost, res.final_cost], np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def median(xs):
     return float(np.median(np.asarray(xs, dtype=np.float64)))
 
@@ -182,16 +201,19 @@ def median(xs):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=1000)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--no-global-ba", action="store_true", help="skip the config-5 global BA section")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     from gslam_b200 import synth
     ba_problem = synth.synth_ba(BA_CAMS, BA_PTS, BA_OBS_PER_PT, seed=42, n_fixed=2)
     cores = os.cpu_count() or 1
 
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none to write")
     if args.impl == "reference":
         if rank != 0:
             return
@@ -201,7 +223,7 @@ def main():
         cpu_path(frames, ba_problem, warm, cores)
         fps, what = cpu_path(frames, ba_problem, steps, cores)
         line = {"impl": "reference", "metric": METRIC, "value": fps, "unit": "frames/s",
-                "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 / fps,
+                "n_gpus": args.gpus, "steps": steps, "warmup": warm, "ms_per_step": 1e3 / fps,
                 "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u8+f64", "data": "synthetic",
                 "config": workload_config(world),
                 "cpu_baseline": {"value": fps, "unit": "frames/s", "cores": cores, "kind": "port",
@@ -258,6 +280,8 @@ def main():
         for k in range(k0, k0 + n):
             step_serial(k)
 
+    res_last = [None]
+
     def run_pipelined(k0, n):
         """n frames from two host threads, like a SLAM's tracking and mapping threads: the tracking thread enqueues extract(k) +
         match(k) (no host synchronisation: the matcher reads the keypoint counts on the device) and orders the mapping stream
@@ -272,7 +296,7 @@ def main():
                     if k is None:
                         return
                     graph_p.reset()
-                    graph_p.solve(ba_cfg)
+                    res_last[0] = graph_p.solve(ba_cfg)
             except Exception as e:
                 err.append(e)
         th = threading.Thread(target=mapper, daemon=True)
@@ -287,26 +311,15 @@ def main():
             raise err[0]
         ctx.wait_for(ctx_m)              # the timing events live on the tracking stream
 
-    def timed_blocks(run, steps):
-        """Repeat [barrier, K steps, barrier] and return the per-block ms (max over ranks each) and the launch count of a block."""
-        blocks, out, launches = None, [], 0
-        k0 = args.warmup
-        b = 0
-        while True:
-            barrier()
-            l0 = ctx.launch_count() + ctx_m.launch_count()
-            ctx.timer_begin()
-            run(k0, steps)
-            ms = ctx.timer_end()
-            torch.cuda.synchronize()
-            launches = ctx.launch_count() + ctx_m.launch_count() - l0
-            out.append(max_over_ranks(ms))
-            k0 += steps
-            b += 1
-            if blocks is None:  # enough repetitions for >= ~0.7 s of timed work and at least 5 blocks (every rank agrees: max'd time)
-                blocks = int(min(60, max(5, math.ceil(700.0 / max(out[0], 1e-3)))))
-            if b >= blocks:
-                return out, launches
+    def timed_block(run, steps):
+        """[barrier, K steps, barrier] -> ms (max over ranks) and the launch count of the block."""
+        barrier()
+        l0 = ctx.launch_count() + ctx_m.launch_count()
+        ctx.timer_begin()
+        run(args.warmup, steps)
+        ms = ctx.timer_end()
+        torch.cuda.synchronize()
+        return max_over_ranks(ms), ctx.launch_count() + ctx_m.launch_count() - l0
 
     feats[1].extract(ring[RING - 1].data_ptr(), W, H, cfg, device_ptr=True, pitch=W)
     run_serial(0, max(3, args.warmup))
@@ -314,10 +327,11 @@ def main():
     ctx.sync(); ctx_m.sync()
     if sampler:
         sampler.mark()
-    ser_ms, ser_launches = timed_blocks(run_serial, args.steps)
-    pip_ms, pip_launches = timed_blocks(run_pipelined, args.steps)
+    ms_serial, ser_launches = timed_block(run_serial, args.steps)
+    ms_pipe, pip_launches = timed_block(run_pipelined, args.steps)
     clocks = sampler.finish() if sampler else None
-    ms_serial, ms_pipe = median(ser_ms), median(pip_ms)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, feats[(args.warmup + args.steps - 1) & 1], graph_p, res_last[0])
 
     # ---- per-stage device timing (CUDA events on the ctx stream) ------------------------------------------------------------
     def time_stage(fn, reps, c=ctx):
@@ -577,9 +591,9 @@ def main():
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms_pipe / args.steps, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "u8+f64", "data": "synthetic",
             "config": workload_config(world),
-            "timing": {"blocks": len(pip_ms), "block_ms_median": ms_pipe, "block_ms_min": min(pip_ms), "block_ms_max": max(pip_ms),
-                       "rule": "each block = exactly --steps steps between barrier+synchronize, CUDA events, max over ranks; median block reported"},
-            "serial": {"value": world * args.steps / (ms_serial * 1e-3), "ms_per_step": ms_serial / args.steps, "blocks": len(ser_ms),
+            "timing": {"blocks": 1, "block_ms": ms_pipe,
+                       "rule": "one block of exactly --steps steps between barrier+synchronize, CUDA events, max over ranks"},
+            "serial": {"value": world * args.steps / (ms_serial * 1e-3), "ms_per_step": ms_serial / args.steps, "blocks": 1,
                        "note": "the same steps on ONE stream (round-1 definition of `value`)", "gpu_launches": int(ser_launches)},
             "clocks": clocks, "gpu_launches": int(pip_launches),
             "e2e": {"value": e2e_pipe_pageable, "unit": "frames/s", "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": int(d2h),
